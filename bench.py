@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            (N>1: launched by torch.distributed.run, one rank per GPU)
   python bench.py --impl reference ...                      (the CPU arm: the oracle port on the host cores)
+  python bench.py ... --dump-outputs DIR                    (also writes the poses of the last timed step, DIR/poses.npy)
 
 A "step" is one Tracker::ExecuteTrackingStep pass (n_corr correspondence iterations x n_update update
 iterations, tracker.cpp:344-361) over this GPU's batch of bodies = ONE launch of the fused kernel k_track.
@@ -64,7 +65,14 @@ def parse_args():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-parity-check", action="store_true")
     ap.add_argument("--no-secondary", action="store_true", help="skip the short runs of the other BASELINE configs")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the poses the last timed step solved (every body of the job, float32) to DIR/poses.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes what the B200 path computed; it does not apply to --impl reference")
+    return args
 
 
 def workload_description(wl, args, per_gpu=None):
@@ -484,6 +492,15 @@ def run_b200(args):
     torch.cuda.synchronize(dev)
     launches = ctx.launch_count - launches0
     barrier()
+    if args.dump_outputs:  # before the e2e and clock loops below move the poses on
+        poses_out = torch.from_numpy(ctx.get_poses()).to(dev)
+        if world > 1:  # equal shards in rank order: the whole job's bodies
+            gathered_out = torch.empty((world * nb, 3, 4), dtype=torch.float32, device=dev)
+            dist.all_gather_into_tensor(gathered_out, poses_out)
+            poses_out = gathered_out
+        if rank == 0:
+            os.makedirs(args.dump_outputs, exist_ok=True)
+            np.save(os.path.join(args.dump_outputs, "poses.npy"), poses_out.cpu().numpy())
     total_ms = sum(a.elapsed_time(b) for a, b in evs)
     t = torch.tensor([total_ms], dtype=torch.float64, device=dev)
     if world > 1:

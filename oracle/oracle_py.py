@@ -7,7 +7,9 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -152,9 +154,19 @@ class Structure(C.Structure):
 _libs = {}
 
 
-def build(native=False):
-    target = "native" if native else "all"
-    subprocess.run(["make", "-C", _HERE, target], check=True, capture_output=True)
+def build():
+    subprocess.run(["make", "-C", _HERE, "all"], check=True, capture_output=True)
+
+
+def _load_native():
+    """Compiles the -O3 -march=native build for this machine's CPU into a temporary directory (the tree may be
+    read-only), loads it and removes the directory again."""
+    d = tempfile.mkdtemp(prefix="m3t_oracle_native-")
+    try:
+        subprocess.run(["make", "-C", _HERE, "native", f"NATIVE_DIR={d}/"], check=True, capture_output=True)
+        return C.CDLL(os.path.join(d, "libm3t_oracle_native.so"))
+    finally:
+        shutil.rmtree(d, ignore_errors=True)
 
 
 def lib(native=False):
@@ -162,11 +174,13 @@ def lib(native=False):
     key = "native" if native else "strict"
     if key in _libs:
         return _libs[key]
-    name = "libm3t_oracle_native.so" if native else "libm3t_oracle.so"
-    path = os.path.join(_HERE, name)
-    if native or not os.path.exists(path):
-        build(native)
-    L = C.CDLL(path)
+    if native:
+        L = _load_native()
+    else:
+        path = os.path.join(_HERE, "libm3t_oracle.so")
+        if not os.path.exists(path):
+            build()
+        L = C.CDLL(path)
     L.orc_region_params_default.argtypes = [C.POINTER(RegionParams)]
     L.orc_depth_params_default.argtypes = [C.POINTER(DepthParams)]
     L.orc_pose_multiply.argtypes = [fp, fp, fp]
